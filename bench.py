@@ -49,7 +49,21 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the C1 / C3 / C5 side results")
     ap.add_argument("--no-parity", action="store_true", help="skip the Acero / oracle checks of the timed workload")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result columns of the last timed step to DIR/<tuple>_<slot>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(out_dir, columns):
+    """columns: {"<tuple>_<slot>": array} of one GROUP BY result.  Written as float64 (COUNT fits exactly), rows ordered by the
+    group key `0_1`: the engines return groups in no particular order, and a fixed order lets two builds be compared row for row."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    order = np.argsort(columns["0_1"], kind="stable")
+    for name, values in columns.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(values)[order].astype(np.float64))
 
 
 def env_rank():
@@ -242,8 +256,10 @@ def run_reference(args):
     assert out.num_rows == N_GROUPS
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        A.c2_filter_groupby(table, K_FILTER, use_threads=True)
+        out = A.c2_filter_groupby(table, K_FILTER, use_threads=True)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {name: out.column(name).to_numpy() for name in out.column_names})
     value = sample * args.steps / dt
     # the reference's DEFAULT executes the declaration single-threaded (FLAGS vectorlized_parallel_execution = false,
     # src/runtime/arrow_io_excutor.cpp:266-270): reported beside the all-threads number
@@ -434,8 +450,9 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(run_step, steps, warmup, hh=None, all_ranks=True):
-        """all_ranks=False: a measurement only this rank takes part in (no barrier, no reduction over the ranks)"""
+    def timed(run_step, steps, warmup, hh=None, all_ranks=True, keep_last=False):
+        """all_ranks=False: a measurement only this rank takes part in (no barrier, no reduction over the ranks);
+        keep_last: the last timed step copies its result columns out (run_step(keep=True))"""
         sync = barrier if all_ranks else torch.cuda.synchronize
         for _ in range(warmup):
             run_step()
@@ -447,8 +464,8 @@ def main():
         e0.record(stream)
         res = None
         kernel_ms, kernel_launches, kernel_bytes, coll_ms = 0.0, 0, 0, 0.0
-        for _ in range(steps):
-            res = run_step()
+        for i in range(steps):
+            res = run_step(keep=True) if keep_last and i == steps - 1 else run_step()
             st = get_stats(hh)
             kernel_ms += st.main_kernel_ms; kernel_launches += st.main_kernel_launches
             kernel_bytes += st.main_kernel_bytes; coll_ms += st.collective_ms
@@ -465,7 +482,9 @@ def main():
                 "kernel_ms": kernel_ms, "kernel_launches": kernel_launches, "kernel_bytes": kernel_bytes, "coll_ms": coll_ms}
 
     # ---- value: device-resident columns ----
-    r = timed(lambda: step(dcols, 1), args.steps, max(args.warmup, 3))
+    r = timed(lambda keep=False: step(dcols, 1, keep=keep), args.steps, max(args.warmup, 3), keep_last=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f"{tup}_{slot}": v for (tup, slot), v in r["res"][2].items()})
     if os.environ.get("BKGPU_BENCH_TRACE"):   # per-rank view of the timed region (stderr)
         sys.stderr.write(f"[rank {rank}] step {r['ms'] / args.steps:.4f} ms  kernel {r['kernel_ms'] / max(r['kernel_launches'], 1):.4f} ms  "
                          f"collective {r['coll_ms'] / args.steps:.4f} ms  launches/step {r['launches'] / args.steps:.1f}\n")

@@ -113,7 +113,6 @@ def test_unsupported_uses_of_strings_are_refused():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(__import__("os").environ.get("BKGPU_UNVERIFIED") != "1", reason="written after round 2's last GPU window: not yet run on a GPU")
 def test_gpu_runs_the_rewritten_fragment():
     """the GPU sees only INT32 codes: the rewritten GROUP BY / MIN / MAX fragment through the C ABI equals the oracle, and decodes to pyarrow's answer"""
     from tests.util import run_both

@@ -1,8 +1,6 @@
 """GPU parity of the lean kernel's FX variant (double sums as fixed-point limbs updated with native 32-bit shared atomics,
 csrc/agg_direct.cuh + csrc/fx.h) against the row-engine oracle, through the C ABI: value distributions that exercise the main / fine /
 exact classes, special values, group counts on both sides of the shared table's capacity, the fused join probe, and agreement with the CAS variant."""
-import os
-
 import numpy as np
 import pytest
 
@@ -153,7 +151,6 @@ def test_fx_fused_join_probe():
     assert stats.main_kernel_name.decode() == NAME
 
 
-@pytest.mark.skipif(os.environ.get("BKGPU_UNVERIFIED") != "1", reason="written after round 2's last GPU window: not yet run on a GPU")
 def test_fx_plan_goes_back_to_cas_when_its_values_do_not_fit_one_scale():
     """a reused plan (bkgpu_reset) whose double column puts most rows on FX's exact path — outliers 1e18 times the bulk dominate the
     sample — launches the CAS kernel from its second request on (the exact-path counter comes back with the counter block)"""

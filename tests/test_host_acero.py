@@ -53,7 +53,6 @@ def test_without_a_gpu_the_plan_fails_loudly(acero_bin, tmp_path):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(os.environ.get("BKGPU_UNVERIFIED") != "1", reason="written after round 2's last GPU window: not yet run on a GPU")
 @pytest.mark.parametrize("batch_rows", [7000, 1 << 20])
 def test_acero_plan_with_the_gpu_fragment_equals_the_oracle(acero_bin, tmp_path, batch_rows):
     cols = datagen.c2_table(0, 200_000, n_groups=77)
